@@ -17,6 +17,10 @@ The same invocation also measures (sub-records under ``configs``, skipped with `
   config 5  Pangu ensemble with 4 members per GPU (32 members on 8 GPUs)      -> configs.ensemble_m4
 each with ms/step, member-steps/s, per-family roofline fractions, fixture verification, and (N = 1) its e2e figure.
 One JSON line on rank 0.
+
+``--dump-outputs DIR`` also writes DIR/state.npy: 2**23 elements (fewer after removing repeats) of the state the last timed
+headline step returned, at flat indices fixed by a seed.  Weights and initial conditions are seeded too, so two builds run
+with the same arguments can be compared element for element.
 """
 from __future__ import annotations
 
@@ -36,6 +40,7 @@ UNIT = "member-steps/s"
 VERIFY_TOL = 1e-3      # per-channel relative L2 on the point sample (north star); block means / RMS in sigma units below
 VERIFY_TOL_SIGMA = 5e-3
 VERIFY_TOL_TENDENCY = 4e-3   # GraphCast: per-channel relative L2 of the network tendency (state = x + 0.1 sigma x tendency); measured 1.4e-3
+DUMP_MAX_VALUES = 1 << 23    # --dump-outputs: 32 MB of float32 at most
 
 
 def _peaks():
@@ -298,7 +303,17 @@ def family_roofline(model, cfg, M, fam_ms, peaks):
     return out, fl, by
 
 
-def bench_model(model: str, M: int, steps: int, warmup: int, d: Dist, e2e: bool = True):
+def output_sample(t, n=DUMP_MAX_VALUES, seed=0):
+    """float32 host copy of `t` flattened and read at up to `n` flat indices: sorted, without repeats, drawn from numpy's
+    default generator seeded with `seed`, so every run and every build with the same arguments samples the same elements."""
+    import numpy as np
+    import torch
+    idx = np.sort(np.random.default_rng(seed).integers(0, t.numel(), n))
+    idx = idx[np.concatenate(([True], idx[1:] != idx[:-1]))]   # np.unique does the same, forty times slower
+    return t.reshape(-1)[torch.from_numpy(idx).to(t.device)].float().cpu().numpy()
+
+
+def bench_model(model: str, M: int, steps: int, warmup: int, d: Dist, e2e: bool = True, dump: bool = False):
     import torch
     from skyrim_b200.engine import launch_count, perturb_ic
     from skyrim_b200.verify import compare_fullsize, load_fixture, summarise
@@ -369,6 +384,7 @@ def bench_model(model: str, M: int, steps: int, warmup: int, d: Dist, e2e: bool 
     launches = launch_count() - launches0
     finite = bool(torch.isfinite(src).all())
     z_first = z[0].clone()
+    last_state = output_sample(src) if dump else None   # the passes below overwrite the rotation buffers
 
     # ---- the same K steps once more with CUDA events around every launch of the dominant family (plain launches: the
     # per-launch events cannot live inside a replayed graph) -> roofline.achieved; its wall time is reported beside it ----
@@ -435,6 +451,8 @@ def bench_model(model: str, M: int, steps: int, warmup: int, d: Dist, e2e: bool 
            "value": d.world * M * 1000.0 / ms_step, "unit": UNIT, "gpu_launches": int(launches), "clocks": clocks,
            "verify": verify, "dominant": dominant, "dominant_launches_per_step": dom[1] / steps,
            "dominant_avg_launch_ms": dom[0] / max(dom[1], 1), "ms_per_step_profiled_pass": ms_profiled}
+    if dump:
+        rec["_last_state"] = last_state
     if e2e:
         sbytes = cfg.n_channels * cfg.nlat * cfg.nlon * 4 * M
         rec["e2e"] = {"value": d.world * M * 1000.0 / e2e_max, "unit": UNIT, "ms_per_step": e2e_max,
@@ -480,7 +498,11 @@ def run_ours(args):
     import torch
     d = Dist(args)
     M = args.members_per_gpu
-    head = bench_model(args.model, M, args.steps, args.warmup, d)
+    head = bench_model(args.model, M, args.steps, args.warmup, d, dump=args.dump_outputs is not None and d.rank == 0)
+    if d.rank == 0 and args.dump_outputs is not None:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "state.npy"), head.pop("_last_state"))
     subs = {}
     if not args.only_headline:
         k = max(3, min(args.steps, 8))
@@ -567,7 +589,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--allow-unverified", action="store_true",
                     help="print the line (verify.ok = false) instead of exiting 3 when the fixture comparison fails")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write DIR/state.npy: a fixed seeded sample (output_sample) of the state the last timed headline "
+                         "step returned on rank 0, float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -185,3 +185,18 @@ def test_bench_traffic_lookup_and_roofline_tables():
     assert abs(fl["total"] - 8.26e12) < 0.2e12 and 28e9 < by["total"] < 36e9   # image-only token stream (12 -> 6 B in proj / mlp)
     fams, fl, by = mod.family_roofline("sfno", sfno_full(), 1, {"sfno_mlp": 5.0}, dict(hbm=6572.0, tensor_sustained=1431.0))
     assert "sfno_mlp" in fams and 2e12 < fl["total"] < 6e12
+
+
+def test_bench_output_sample_is_fixed_by_the_seed():
+    """bench.py --dump-outputs: the same distinct, sorted elements of a state larger than the sample on every call, as
+    float32, within 64 MB"""
+    import importlib.util, os
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(root, "bench.py"))
+    mod = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mod)
+    t = torch.arange(2 ** 24, dtype=torch.float64).reshape(4, 2 ** 11, 2 ** 11)   # value = flat index, exact in float32
+    a, b = mod.output_sample(t), mod.output_sample(t)
+    assert a.dtype == np.float32 and a.ndim == 1 and np.array_equal(a, b) and a.nbytes <= 64 * 2 ** 20
+    assert mod.DUMP_MAX_VALUES // 2 < len(a) <= mod.DUMP_MAX_VALUES and (np.diff(a) > 0).all()
+    assert not np.array_equal(mod.output_sample(t, seed=1), a)

@@ -1,6 +1,7 @@
 """World-size-2 gloo tests of the host-side multi-GPU logic (no GPU): the single weight-arena
 broadcast and the member partition (SURVEY.md §8(e))."""
 import os
+import socket
 
 import numpy as np
 import pytest
@@ -11,6 +12,13 @@ import torch.multiprocessing as mp
 from skyrim_b200.config import pangu_small
 from skyrim_b200.ensemble import broadcast_arena, mean_and_spread, member_range
 from skyrim_b200.weights import make_pangu_weights, pangu_param_shapes
+
+
+def _free_port():
+    """a port no other process on the host holds right now: the rendezvous must not depend on a fixed one being free"""
+    with socket.socket(socket.AF_INET, socket.SOCK_STREAM) as s:
+        s.bind(("127.0.0.1", 0))
+        return s.getsockname()[1]
 
 
 def _worker(rank, world, port, q):
@@ -34,7 +42,7 @@ def _worker(rank, world, port, q):
 
 
 def test_weight_broadcast_and_member_partition():
-    world, port = 2, 29517
+    world, port = 2, _free_port()
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     ps = [ctx.Process(target=_worker, args=(r, world, port, q)) for r in range(world)]
@@ -76,7 +84,7 @@ def _worker_graphcast(rank, world, port, q):
 
 
 def test_graphcast_arena_with_graph_tables_broadcasts():
-    world, port = 2, 29519
+    world, port = 2, _free_port()
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     ps = [ctx.Process(target=_worker_graphcast, args=(r, world, port, q)) for r in range(world)]

@@ -1,5 +1,7 @@
 """GraphCast host side on the CPU: the icosahedral multimesh and the grid<->mesh edge sets (skyrim_b200/icomesh.py), the
 oracle (oracle/graphcast_ref.py) against its committed fp64 fixture, and the algebraic rewrites the CUDA engine relies on."""
+import os
+
 import numpy as np
 import pytest
 import torch
@@ -130,7 +132,7 @@ def test_forcing_formulas():
 # -- oracle -----------------------------------------------------------------------------------------------------------
 def test_oracle_matches_committed_fp64_fixture(small):
     cfg, g, w, x = small
-    fix = np.load("tests/golden/graphcast_41x96_seed0.npz")
+    fix = np.load(os.path.join(os.path.dirname(__file__), "golden", "graphcast_41x96_seed0.npz"))
     y = GraphCastRef(cfg, w, g).step(x, T0).numpy()
     assert y.shape == (166, 41, 96)
     err = rel_err_per_channel(y[83:165, ::2, ::3], fix["prog_sample"])
