@@ -27,7 +27,7 @@ extern "C" {
 
 #define SKY_ABI_VERSION 1
 
-enum { SKY_MODEL_PANGU6 = 1, SKY_MODEL_SFNO73 = 2, SKY_MODEL_GRAPHCAST = 3 };
+enum { SKY_MODEL_PANGU6 = 1, SKY_MODEL_SFNO73 = 2, SKY_MODEL_GRAPHCAST = 3, SKY_MODEL_AFNO26 = 4 };
 enum { SKY_OK = 0, SKY_ERR_ARG = -1, SKY_ERR_CUDA = -2, SKY_ERR_STATE = -3, SKY_ERR_NOMEM = -4 };
 
 /* Pangu-Weather 6-h operator shape (patch (2,4,4) and window (2,6,12) are fixed).
@@ -82,6 +82,28 @@ typedef struct {
  *   graph.m2g.senders (3 * nlat * nlon, k-major: edge k of grid point g at k * n_grid + g), graph.m2g.edge_feat (3 * n_grid, 4),
  *   graph.grid.coslat (nlat), graph.grid.sinlon / .coslon (nlon)
  * (skyrim_b200/weights.py::graphcast_param_shapes, skyrim_b200/icomesh.py::graph_arena_entries build exactly this set). */
+
+/* FourCastNet v1 (AFNONet) operator shape; replaces the hyper-parameters earth2mip's networks.fcn package reads
+ * (/root/reference/skyrim/core/models/fourcastnet.py:build_model). */
+typedef struct {
+  int32_t nlat, nlon;      /* 720, 1440 (no south-pole row) */
+  int32_t n_channels;      /* 26 */
+  int32_t patch;           /* 8 */
+  int32_t embed;           /* 768 */
+  int32_t depth;           /* 12 */
+  int32_t num_blocks;      /* 8 spectral blocks of embed / num_blocks = 96 */
+  int32_t mlp_ratio;       /* 4 */
+  float sparsity;          /* softshrink lambda, 0.01 */
+  float hard_thresholding_fraction;  /* 1.0 */
+  float ln_eps;            /* 1e-6 */
+} sky_afno_config_t;
+/* Arena entries of a FourCastNet model (all fp32, upstream names):
+ *   norm.mean, norm.std (n_channels), patch_embed.proj.weight (embed, n_channels, 8, 8), patch_embed.proj.bias (embed),
+ *   pos_embed (1, (nlat / 8) * (nlon / 8), embed), head.weight (n_channels * 64, embed) [columns (p1, p2, c)], and per block i
+ *   blocks.<i>.norm1.weight / .bias, blocks.<i>.norm2.weight / .bias (embed), blocks.<i>.filter.w1 / .w2 (2, num_blocks, 96, 96)
+ *   [re / im, block, in, out], blocks.<i>.filter.b1 / .b2 (2, num_blocks, 96), blocks.<i>.mlp.fc1.weight (mlp_ratio * embed,
+ *   embed), .fc1.bias, blocks.<i>.mlp.fc2.weight (embed, mlp_ratio * embed), .fc2.bias
+ * (skyrim_b200/weights.py::fcn_param_shapes builds exactly this set). */
 
 /* one named fp32 tensor inside a flat weight arena */
 typedef struct {

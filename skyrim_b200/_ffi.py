@@ -18,6 +18,7 @@ DEV_LIB_PATH = Path(__file__).resolve().parent / "libskyrim_b200_dev.so"
 SKY_MODEL_PANGU6 = 1
 SKY_MODEL_SFNO73 = 2
 SKY_MODEL_GRAPHCAST = 3
+SKY_MODEL_AFNO26 = 4
 
 
 class SkyError(RuntimeError):
@@ -40,6 +41,12 @@ class GraphCastConfigC(C.Structure):
     _fields_ = [("nlat", C.c_int32), ("nlon", C.c_int32), ("n_mesh", C.c_int32), ("n_mesh_edges", C.c_int32),
                 ("n_g2m_edges", C.c_int32), ("latent", C.c_int32), ("layers", C.c_int32), ("n_state", C.c_int32),
                 ("n_prog", C.c_int32), ("n_static", C.c_int32), ("dt_hours", C.c_int32), ("ln_eps", C.c_float)]
+
+
+class AFNOConfigC(C.Structure):
+    _fields_ = [("nlat", C.c_int32), ("nlon", C.c_int32), ("n_channels", C.c_int32), ("patch", C.c_int32),
+                ("embed", C.c_int32), ("depth", C.c_int32), ("num_blocks", C.c_int32), ("mlp_ratio", C.c_int32),
+                ("sparsity", C.c_float), ("hard_thresholding_fraction", C.c_float), ("ln_eps", C.c_float)]
 
 
 class ParamDesc(C.Structure):

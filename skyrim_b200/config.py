@@ -1,4 +1,5 @@
-"""Shape configuration of the step operators on the hot path (Pangu-Weather, FourCastNet-v2 SFNO, GraphCast).
+"""Shape configuration of the step operators on the hot path (Pangu-Weather, FourCastNet-v2 SFNO, GraphCast,
+FourCastNet v1 AFNO).
 
 The reference carries no architecture description of its own (SURVEY.md §0): the
 arithmetic lives in ONNX graphs / earth2mip modules it downloads.  The numbers below
@@ -186,3 +187,72 @@ def graphcast_full() -> GraphCastConfig:
 
 def graphcast_small(nlat: int = 41, nlon: int = 96, mesh_levels: int = 2, latent: int = 512, layers: int = 2) -> GraphCastConfig:
     return GraphCastConfig(nlat=nlat, nlon=nlon, mesh_levels=mesh_levels, latent=latent, layers=layers)
+
+
+# ----------------------------------------------------------------------------------------
+# FourCastNet v1 (AFNO backbone)
+# ----------------------------------------------------------------------------------------
+# /root/reference/skyrim/core/models/fourcastnet.py:8-11
+FCN_CHANNELS = ["u10m", "v10m", "t2m", "sp", "msl", "t850", "u1000", "v1000", "z1000", "u850", "v850", "z850", "u500",
+                "v500", "z500", "t500", "z50", "r500", "r850", "tcwv", "u100m", "v100m", "u250", "v250", "z250", "t250"]
+
+
+@dataclass(frozen=True)
+class FCNConfig:
+    """FourCastNet v1 AFNONet (SURVEY.md Appendix D): 8x8 patch embedding, `depth` blocks of LayerNorm -> AFNO2D
+    filter (double skip) -> LayerNorm -> GELU MLP, linear head.  The grid has no south-pole row (720 x 1440)."""
+    nlat: int = 720
+    nlon: int = 1440
+    n_channels: int = 26
+    patch: int = 8
+    embed: int = 768
+    depth: int = 12
+    num_blocks: int = 8
+    mlp_ratio: int = 4
+    sparsity: float = 0.01                     # softshrink lambda
+    hard_thresholding_fraction: float = 1.0
+    ln_eps: float = 1e-6
+
+    @property
+    def h(self):
+        return self.nlat // self.patch
+
+    @property
+    def w(self):
+        return self.nlon // self.patch
+
+    @property
+    def tokens(self):
+        return self.h * self.w
+
+    @property
+    def block_size(self):
+        return self.embed // self.num_blocks
+
+    @property
+    def kept(self):
+        return int((self.h // 2 + 1) * self.hard_thresholding_fraction)
+
+    @property
+    def h_range(self):
+        """H-frequency rows the filter processes: upstream's slice [total - kept : total + kept] (clipped to h)"""
+        total = self.h // 2 + 1
+        return total - self.kept, min(total + self.kept, self.h)
+
+    @property
+    def kw(self):
+        """W-modes the filter processes: upstream's slice [:kept] of the w // 2 + 1 rfft modes"""
+        return min(self.kept, self.w // 2 + 1)
+
+    def validate(self):
+        assert self.nlat % self.patch == 0 and self.nlon % self.patch == 0, "the grid must tile by the patch"
+        assert self.embed % self.num_blocks == 0
+        return self
+
+
+def fcn_full() -> FCNConfig:
+    return FCNConfig().validate()
+
+
+def fcn_small(nlat: int = 48, nlon: int = 96, depth: int = 2) -> FCNConfig:
+    return FCNConfig(nlat=nlat, nlon=nlon, depth=depth).validate()

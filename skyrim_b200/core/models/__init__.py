@@ -2,6 +2,7 @@
 two step operators the north star names plus GraphCast (BASELINE config 4); the other reference wrappers
 (fourcastnet, dlwp, fuxi, fengwu) are not part of this path."""
 from .base import GlobalModel, GlobalPrediction, GlobalPredictionRollout  # noqa: F401
+from .fourcastnet import FourcastnetModel  # noqa: F401  (not in MODELS yet: the facade's model list is pinned)
 from .fourcastnet_v2 import FourcastnetV2Model
 from .graphcast import GraphcastModel
 from .pangu import PanguModel

@@ -20,7 +20,8 @@ void set_error(const char* fmt, ...);
 // kernel families, used for per-kernel CUDA-event timing (bench.py roofline) and launch counting
 enum KTag { KT_EMBED = 0, KT_QKV, KT_ATTN, KT_PROJ, KT_FC1, KT_FC2, KT_MLP, KT_DOWN, KT_UP, KT_RECOVER, KT_COPY,
             KT_SFNO_ENC, KT_SFNO_SHT, KT_SFNO_SPEC, KT_SFNO_ISHT, KT_SFNO_MLP, KT_SFNO_DEC, KT_SFNO_MISC,
-            KT_GC_FEAT, KT_GC_HIDDEN, KT_GC_LN, KT_GC_TABLE, KT_GC_AGG, KT_GC_OUT, KT_GC_MISC, KT_COUNT };
+            KT_GC_FEAT, KT_GC_HIDDEN, KT_GC_LN, KT_GC_TABLE, KT_GC_AGG, KT_GC_OUT, KT_GC_MISC,
+            KT_FCN_EMBED, KT_FCN_LN, KT_FCN_SPEC, KT_FCN_MLP, KT_FCN_HEAD, KT_COUNT };
 const char* ktag_name(int tag);
 
 struct ParamView {
@@ -42,7 +43,8 @@ struct Engine {
   // max |value| per class in range_dev[8] (read back with debug_copy "range").  The tensor cores take fp16 operands (5
   // exponent bits): with real checkpoints the caller runs the first step of a rollout guarded and refuses anything > 3e4.
   // Slots: 0 token images (LN outputs), 1 q/k/v, 2 attention output, 3 down / up-sampled images (Pangu);
-  //        4 pixel images, 5 hidden images, 6 spectral images (SFNO).
+  //        4 pixel images, 5 hidden images, 6 spectral images (SFNO).  FourCastNet scans its LN2 rows (0) and its MLP
+  //        hidden rows (5); its spectral filter runs in fp32 and has no fp16 image.
   int range_guard = 0;
   float* range_dev = nullptr;
   int range_scan(int slot, const void* img, size_t bytes, cudaStream_t st);   // no-op unless range_guard
@@ -91,6 +93,7 @@ struct Engine {
 Engine* make_pangu_engine(const sky_pangu_config_t& cfg, int device);
 Engine* make_sfno_engine(const sky_sfno_config_t& cfg, int device);
 Engine* make_graphcast_engine(const sky_graphcast_config_t& cfg, int device);
+Engine* make_fcn_engine(const sky_afno_config_t& cfg, int device);
 int toa_radiation_launch(float* out, int nlat, int nlon, double unix_seconds, cudaStream_t st);
 
 }  // namespace sky

@@ -104,7 +104,8 @@ int Engine::range_scan(int slot, const void* img, size_t bytes, cudaStream_t st)
 const char* ktag_name(int t) {
   static const char* n[KT_COUNT] = {"embed", "qkv", "attn", "proj", "fc1", "fc2", "mlp", "down", "up", "recover", "copy",
                                     "sfno_enc", "sfno_sht", "sfno_spec", "sfno_isht", "sfno_mlp", "sfno_dec", "sfno_misc",
-                                    "gc_feat", "gc_hidden", "gc_ln", "gc_table", "gc_agg", "gc_out", "gc_misc"};
+                                    "gc_feat", "gc_hidden", "gc_ln", "gc_table", "gc_agg", "gc_out", "gc_misc",
+                                    "fcn_embed", "fcn_ln", "fcn_spec", "fcn_mlp", "fcn_head"};
   return t >= 0 && t < KT_COUNT ? n[t] : "?";
 }
 
@@ -281,6 +282,9 @@ int sky_model_create(sky_model_t** out, int kind, const void* cfg, size_t cfg_by
   } else if (kind == SKY_MODEL_GRAPHCAST) {
     if (cfg_bytes != sizeof(sky_graphcast_config_t)) { set_error("bad config size"); return SKY_ERR_ARG; }
     e = make_graphcast_engine(*static_cast<const sky_graphcast_config_t*>(cfg), device);
+  } else if (kind == SKY_MODEL_AFNO26) {
+    if (cfg_bytes != sizeof(sky_afno_config_t)) { set_error("bad config size"); return SKY_ERR_ARG; }
+    e = make_fcn_engine(*static_cast<const sky_afno_config_t*>(cfg), device);
   } else {
     set_error("unknown model kind %d", kind);
     return SKY_ERR_ARG;

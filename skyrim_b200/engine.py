@@ -11,7 +11,7 @@ from collections import OrderedDict
 import numpy as np
 
 from . import _ffi
-from .config import GraphCastConfig, PanguConfig, SFNOConfig
+from .config import FCNConfig, GraphCastConfig, PanguConfig, SFNOConfig
 
 ARENA_ALIGN = 64  # floats (256 B)
 
@@ -57,6 +57,14 @@ def _graphcast_cfg_c(cfg: GraphCastConfig, graph) -> _ffi.GraphCastConfigC:
     return c
 
 
+def _afno_cfg_c(cfg: FCNConfig) -> _ffi.AFNOConfigC:
+    c = _ffi.AFNOConfigC()
+    c.nlat, c.nlon, c.n_channels, c.patch, c.embed = cfg.nlat, cfg.nlon, cfg.n_channels, cfg.patch, cfg.embed
+    c.depth, c.num_blocks, c.mlp_ratio = cfg.depth, cfg.num_blocks, cfg.mlp_ratio
+    c.sparsity, c.hard_thresholding_fraction, c.ln_eps = cfg.sparsity, cfg.hard_thresholding_fraction, cfg.ln_eps
+    return c
+
+
 class StepEngine:
     """One 6-h step operator resident on one GPU."""
 
@@ -79,6 +87,8 @@ class StepEngine:
                 graph = build_graph(cfg.nlat, cfg.nlon, cfg.mesh_levels, cfg.radius_frac)
             self.graph = graph
             kind, cc = _ffi.SKY_MODEL_GRAPHCAST, _graphcast_cfg_c(cfg, graph)
+        elif isinstance(cfg, FCNConfig):
+            kind, cc = _ffi.SKY_MODEL_AFNO26, _afno_cfg_c(cfg)
         else:
             raise TypeError(cfg)
         self.n_channels = cfg.n_channels

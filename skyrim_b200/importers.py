@@ -362,6 +362,48 @@ def sfno_from_checkpoint(weights_path: str, means_path: str | None = None, stds_
     return cfg, res
 
 
+def fcn_from_checkpoint(weights_path: str, means_path: str, stds_path: str):
+    """FourCastNet v1 checkpoint (torch.load state dict, top level or under "model_state", "module." prefix optional)
+    + global_means.npy / global_stds.npy -> (FCNConfig, parameter dict).  Hyper-parameters come from the tensor shapes."""
+    import torch
+    from .config import FCNConfig
+    from .weights import fcn_param_shapes
+    ck = torch.load(weights_path, map_location="cpu", weights_only=False)
+    sd = ck.get("model_state", ck) if isinstance(ck, dict) else ck
+    sd = {(k[7:] if k.startswith("module.") else k): v.detach().cpu().float().numpy() for k, v in sd.items()}
+    if "patch_embed.proj.weight" not in sd:
+        raise KeyError(f"not a FourCastNet (AFNONet) state dict: no 'patch_embed.proj.weight'; keys start {list(sd)[:8]}")
+    E, C, p, _ = sd["patch_embed.proj.weight"].shape
+    T = sd["pos_embed"].shape[1]
+    depth = 0
+    while f"blocks.{depth}.norm1.weight" in sd:
+        depth += 1
+    _, nb, bs, _ = sd["blocks.0.filter.w1"].shape
+    mlp_ratio = sd["blocks.0.mlp.fc1.weight"].shape[0] // E
+    # the grid is not stored; the token count fixes it for the 1:2 aspect ratio of the global lat-lon grid
+    w = int(round(np.sqrt(2 * T)))
+    if w * (w // 2) != T or w % 2:
+        raise ValueError(f"pos_embed has {T} tokens: not an h x 2h token grid")
+    cfg = FCNConfig(nlat=p * (w // 2), nlon=p * w, n_channels=C, patch=p, embed=E, depth=depth, num_blocks=nb,
+                    mlp_ratio=mlp_ratio)
+    stats = {}
+    for key, path in (("norm.mean", means_path), ("norm.std", stds_path)):
+        a = np.squeeze(np.load(path))
+        if a.shape != (C,):
+            raise ValueError(f"{os.path.basename(path)} has shape {np.load(path).shape}: expected {C} values after squeeze")
+        stats[key] = a.astype(np.float32)
+    res = OrderedDict()
+    for k, shp in fcn_param_shapes(cfg).items():
+        a = stats[k] if k in stats else sd.get(k)
+        if a is None:
+            raise KeyError(f"checkpoint lacks '{k}'")
+        a = np.ascontiguousarray(a, dtype=np.float32)
+        if a.shape != tuple(shp):
+            raise ValueError(f"{k}: checkpoint shape {a.shape} != expected {tuple(shp)}")
+        res[k] = a
+    return cfg, res
+
+
 # ----------------------------------------------------------------------------------------
 def check_fp16_range(weights, limit: float = 3.0e4):
     """The tensor cores receive fp16 operands (5 exponent bits): refuse weights whose magnitude would overflow, and report
@@ -386,6 +428,11 @@ def load_real_weights(model: str, path: str):
         check_fp16_range(w)
         return None, w
     d = path if os.path.isdir(path) else os.path.dirname(path)
+    if model == "fcn":
+        wp = path if os.path.isfile(path) else os.path.join(d, "weights.tar")
+        cfg, w = fcn_from_checkpoint(wp, os.path.join(d, "global_means.npy"), os.path.join(d, "global_stds.npy"))
+        check_fp16_range(w)
+        return cfg, w
     wp = path if os.path.isfile(path) else os.path.join(d, "weights.tar")
     mp, sp = os.path.join(d, "global_means.npy"), os.path.join(d, "global_stds.npy")
     cfg, w = sfno_from_checkpoint(wp, mp if os.path.exists(mp) else None, sp if os.path.exists(sp) else None)

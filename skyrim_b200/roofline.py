@@ -3,7 +3,7 @@ object and DESIGN.md use; derivation in SURVEY.md §8(d)).  FLOPs are 2*MAC of t
 contractions; bytes are the mandatory HBM traffic of the family's fused kernel."""
 from __future__ import annotations
 
-from .config import PanguConfig, SFNOConfig
+from .config import FCNConfig, PanguConfig, SFNOConfig
 
 WIN_TOK = 144
 
@@ -172,3 +172,38 @@ def graphcast_bytes(cfg, graph=None) -> dict:
     b["gc_out"] = n["Ng"] * 2.0 * L + plane * 2 * cfg.n_prog                                    # hidden in; x_t in, x_{t+1} out
     b["total"] = sum(b.values())
     return b
+
+
+def fcn_flops(cfg: FCNConfig, batch: int = 1) -> dict:
+    """FourCastNet v1 per step, by kernel family of csrc/fcn_engine.cu (fcn_ln does no contraction)"""
+    M = batch * cfg.tokens
+    E, K = cfg.embed, cfg.n_channels * cfg.patch ** 2
+    lo, hi = cfg.h_range
+    nk, kw, h, w = hi - lo, cfg.kw, cfg.h, cfg.w
+    dft_w = 2 * (2.0 * batch * h * E * w * 2 * kw)                   # forward + inverse, real x complex
+    dft_h = 2 * (8.0 * batch * kw * E * h * nk)                      # forward + inverse, complex
+    block_mlp = 2 * (2.0 * batch * nk * kw * E * 2 * 2 * cfg.block_size)
+    f = dict(fcn_embed=2.0 * M * K * E, fcn_head=2.0 * M * E * K, fcn_ln=0.0,
+             fcn_mlp=cfg.depth * 2 * (2.0 * M * E * cfg.mlp_ratio * E), fcn_spec=cfg.depth * (dft_w + dft_h + block_mlp))
+    f["total"] = sum(f.values())
+    return f
+
+
+def fcn_bytes(cfg: FCNConfig, batch: int = 1) -> dict:
+    """Mandatory HBM bytes per step and family for the data flow of csrc/fcn_engine.cu (fp32 token stream x, fp32 LN1
+    output u, fp16 LN2 rows, fp16 hidden rows, complex fp32 spectra; weights counted once as fp16 images)."""
+    M = batch * cfg.tokens
+    E, C, hid = cfg.embed, cfg.n_channels, cfg.mlp_ratio * cfg.embed
+    lo, hi = cfg.h_range
+    nk, kw, h = hi - lo, cfg.kw, cfg.h
+    state = 4.0 * batch * C * cfg.nlat * cfg.nlon
+    spec_h = 8.0 * batch * kw * E * (h + nk)                         # one H-DFT pass: read + write
+    f = dict(fcn_embed=state + 4.0 * M * E + 2.0 * E * C * 64,
+             fcn_head=4.0 * M * E + state + 2.0 * E * C * 64,
+             fcn_ln=cfg.depth * (4.0 * M * E * 2 + 4.0 * M * E + 2.0 * M * E),
+             fcn_mlp=cfg.depth * (2.0 * M * E + 2.0 * M * hid + 2.0 * 2 * E * hid + 2.0 * M * hid + 4.0 * M * E * 2),
+             fcn_spec=cfg.depth * (4.0 * M * E + 8.0 * batch * h * kw * E                 # forward W-DFT
+                                   + 2 * spec_h + 2 * 8.0 * batch * nk * kw * E           # H-DFTs, block MLP
+                                   + 8.0 * batch * h * kw * E + 4.0 * M * E * 3))          # inverse W-DFT + skips
+    f["total"] = sum(f.values())
+    return f

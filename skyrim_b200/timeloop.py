@@ -16,7 +16,7 @@ from dataclasses import dataclass
 
 import numpy as np
 
-from .config import FCNV2_CHANNELS, GRAPHCAST_CHANNELS, PANGU_CHANNELS
+from .config import FCN_CHANNELS, FCNV2_CHANNELS, FCNConfig, GRAPHCAST_CHANNELS, PANGU_CHANNELS
 
 
 @dataclass
@@ -34,6 +34,13 @@ def equiangular_grid(nlat: int = 721, nlon: int = 1440) -> Grid:
     return Grid(lat=np.linspace(90.0, -90.0, nlat).tolist(), lon=(np.arange(nlon) * (360.0 / nlon)).tolist())
 
 
+def poleless_grid(nlat: int = 720, nlon: int = 1440) -> Grid:
+    """FourCastNet v1's grid (fourcastnet.py:16-19): lat = 90 - 0.25 i for i < 720 (the south-pole row is dropped),
+    lon 0 .. 359.75; at other sizes the spacing is 180 / nlat so that the same rows of the 721-row grid are kept."""
+    d = 180.0 / nlat
+    return Grid(lat=(90.0 - d * np.arange(nlat)).tolist(), lon=(np.arange(nlon) * (360.0 / nlon)).tolist())
+
+
 class _EngineTimeLoop:
     n_history_levels = 1
     time_step = datetime.timedelta(hours=6)
@@ -46,7 +53,8 @@ class _EngineTimeLoop:
         self.device = torch.device("cuda", engine.device)
         self.in_channel_names = list(self.channel_names)
         self.out_channel_names = list(self.channel_names)
-        self.grid = equiangular_grid(engine.cfg.nlat, engine.cfg.nlon)
+        cfg = engine.cfg
+        self.grid = poleless_grid(cfg.nlat, cfg.nlon) if isinstance(cfg, FCNConfig) else equiangular_grid(cfg.nlat, cfg.nlon)
         self._dev_in = None
         self._dev_out = None
         self._host_out = None
@@ -141,6 +149,10 @@ class PanguTimeLoop(_EngineTimeLoop):
 
 class SFNOTimeLoop(_EngineTimeLoop):
     channel_names = FCNV2_CHANNELS
+
+
+class FCNTimeLoop(_EngineTimeLoop):
+    channel_names = FCN_CHANNELS
 
 
 class GraphcastStepper:

@@ -12,20 +12,21 @@ import numpy as np
 GOLDEN_DIR = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
 
 
-def load_fixture(model: str):
-    path = os.path.join(GOLDEN_DIR, f"{model}_721x1440_seed0.npz")
+def load_fixture(model: str, nlat: int = 721):
+    path = os.path.join(GOLDEN_DIR, f"{model}_{nlat}x1440_seed0.npz")
     if not os.path.exists(path):
         raise FileNotFoundError(f"{path} missing: run tools/make_golden_full.py {model}")
     return np.load(path)
 
 
-def compare_fullsize(y, fx) -> dict:
-    """y: (C, 721, 1440) torch tensor (any device) or ndarray.  Returns per-channel error vectors:
+def compare_fullsize(y, fx, last_row: int = 720) -> dict:
+    """y: (C, 721, 1440) torch tensor (any device) or ndarray (FourCastNet: (C, 720, 1440) with last_row=719).
+    Returns per-channel error vectors:
       rel      ||y_s - ref_s||_2 / ||ref_s||_2 over the strided point sample (north-star metric, sampled)
       nrm      RMS(y_s - ref_s) / std_c            (in units of the channel's standard deviation: stricter
                                                     for channels whose mean dominates their norm)
       block    max |blockmean16x16(y) - ref| / std_c  over ALL pixels of rows 0..719 (a wrong tile shows here)
-      last     max |y[720, ::4] - ref| / std_c
+      last     max |y[last_row, ::4] - ref| / std_c
       norm     | ||y||_2 / ||ref||_2 - 1 |
     """
     import torch
@@ -42,7 +43,7 @@ def compare_fullsize(y, fx) -> dict:
     nrm = d.pow(2).mean(dim=(1, 2)).sqrt() / std
     blk = t[:, :720].double().reshape(C, 45, 16, 90, 16).mean(dim=(2, 4))
     block = (blk - ref_b).abs().amax(dim=(1, 2)) / std
-    last = (t[:, 720, ::4].double() - ref_l).abs().amax(dim=1) / std
+    last = (t[:, last_row, ::4].double() - ref_l).abs().amax(dim=1) / std
     norm = (t.double().pow(2).sum(dim=(1, 2)).sqrt() / f64(fx["y_norm"]) - 1.0).abs()
     out = {k: v.cpu().numpy() for k, v in dict(rel=rel, nrm=nrm, block=block, last=last, norm=norm).items()}
     out["finite"] = bool(torch.isfinite(t).all())

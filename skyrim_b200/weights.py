@@ -17,7 +17,7 @@ from collections import OrderedDict
 
 import numpy as np
 
-from .config import PRESSURE_LEVELS, GraphCastConfig, PanguConfig, SFNOConfig
+from .config import PRESSURE_LEVELS, FCNConfig, GraphCastConfig, PanguConfig, SFNOConfig
 
 G0 = 9.80665
 
@@ -364,3 +364,64 @@ def synthetic_graphcast_state(cfg: GraphCastConfig, seed: int = 0) -> np.ndarray
     x1 = x0 + np.float32(0.1) * (x1 - mu[:, None, None])
     x0[-1], x1[-1] = mu[-1], mu[-1]
     return np.concatenate([x0, x1], axis=0)
+
+
+# ----------------------------------------------------------------------------------------
+# FourCastNet v1 (AFNO); upstream parameter names (NVlabs FourCastNet AFNONet state dict)
+# ----------------------------------------------------------------------------------------
+def fcn_param_shapes(cfg: FCNConfig) -> "OrderedDict[str, tuple]":
+    E, C, p, nb, bs = cfg.embed, cfg.n_channels, cfg.patch, cfg.num_blocks, cfg.block_size
+    s = OrderedDict()
+    s["norm.mean"] = (C,)
+    s["norm.std"] = (C,)
+    s["patch_embed.proj.weight"] = (E, C, p, p)
+    s["patch_embed.proj.bias"] = (E,)
+    s["pos_embed"] = (1, cfg.tokens, E)
+    for i in range(cfg.depth):
+        b = f"blocks.{i}."
+        s[b + "norm1.weight"] = (E,)
+        s[b + "norm1.bias"] = (E,)
+        s[b + "filter.w1"] = (2, nb, bs, bs)
+        s[b + "filter.b1"] = (2, nb, bs)
+        s[b + "filter.w2"] = (2, nb, bs, bs)
+        s[b + "filter.b2"] = (2, nb, bs)
+        s[b + "norm2.weight"] = (E,)
+        s[b + "norm2.bias"] = (E,)
+        s[b + "mlp.fc1.weight"] = (cfg.mlp_ratio * E, E)
+        s[b + "mlp.fc1.bias"] = (cfg.mlp_ratio * E,)
+        s[b + "mlp.fc2.weight"] = (E, cfg.mlp_ratio * E)
+        s[b + "mlp.fc2.bias"] = (E,)
+    s["head.weight"] = (C * p * p, E)
+    return s
+
+
+def make_fcn_weights(cfg: FCNConfig, seed: int = 0) -> "OrderedDict[str, np.ndarray]":
+    """Synthetic AFNONet parameters.  Linear layers are variance preserving (std 0.9/sqrt(fan_in)); the spectral block
+    MLP uses upstream's initialisation scale (0.02 * N(0, 1)), which leaves a sizeable share of the kept modes inside
+    the softshrink dead band (tests/test_fcn_cpu.py checks the share)."""
+    from .config import FCN_CHANNELS
+    out = OrderedDict()
+    mu, sd = channel_stats(FCN_CHANNELS)
+    for name, shape in fcn_param_shapes(cfg).items():
+        if name == "norm.mean":
+            a = mu
+        elif name == "norm.std":
+            a = sd
+        elif name.endswith(("norm1.weight", "norm2.weight")):
+            g, b = _ln(seed, name[:-7], shape[0])
+            out[name], out[name[:-6] + "bias"] = g, b
+            continue
+        elif name.endswith(("norm1.bias", "norm2.bias")):
+            continue
+        elif ".filter." in name:
+            a = np.float32(0.02) * _rng(seed, name).standard_normal(shape, dtype=np.float32)
+        elif name == "pos_embed":
+            a = _tn(seed, name, shape, std=0.1)
+        elif name.endswith(".bias"):
+            a = _tn(seed, name, shape, std=0.02)
+        elif name == "patch_embed.proj.weight":
+            a = _tn(seed, name, shape, std=0.9 / np.sqrt(np.prod(shape[1:])))
+        else:
+            a = _tn(seed, name, shape, std=0.9 / np.sqrt(shape[-1]))
+        out[name] = np.ascontiguousarray(a, dtype=np.float32)
+    return OrderedDict((k, out[k]) for k in fcn_param_shapes(cfg))

@@ -14,6 +14,18 @@ from oracle.pangu_ref import PanguRef
 out = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
 os.makedirs(out, exist_ok=True)
 ONLY_GRAPHCAST = "--graphcast" in sys.argv   # leave the Pangu / SFNO fixtures untouched
+ONLY_FCN = "--fcn" in sys.argv               # write only the FourCastNet fixture
+if ONLY_FCN:
+    from skyrim_b200.config import fcn_small, FCN_CHANNELS
+    from skyrim_b200.weights import make_fcn_weights
+    from oracle.afno_ref import FCNRef
+    fcfg = fcn_small(48, 96, 2)
+    fx0 = synthetic_state(FCN_CHANNELS, fcfg.nlat, fcfg.nlon, 0)
+    fy = FCNRef(fcfg, make_fcn_weights(fcfg, 0), torch.float64).step(fx0).numpy()
+    np.savez_compressed(os.path.join(out, "fcn_48x96_seed0.npz"), x0_sample=fx0[:, ::8, ::16].astype(np.float32),
+                        y_sample=fy[:, ::5, ::12], y_norm=np.sqrt((fy ** 2).sum(axis=(1, 2))), y_mean=fy.mean(axis=(1, 2)))
+    print("wrote", os.path.join(out, "fcn_48x96_seed0.npz"))
+    sys.exit(0)
 if not ONLY_GRAPHCAST:
     cfg = pangu_small(41, 96)
     w = make_pangu_weights(cfg, 0)

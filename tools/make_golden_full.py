@@ -2,6 +2,8 @@
 
     python tools/make_golden_full.py pangu      # ~5 min on 8 host threads, ~20 GB RAM
     python tools/make_golden_full.py sfno       # E=384, L=8: ~10 min
+    python tools/make_golden_full.py fcn        # FourCastNet v1 (AFNO), 720 x 1440, 12 blocks: writes fcn_720x1440_seed0.npz,
+                                                # y_last = the last (720th) row
     python tools/make_golden_full.py graphcast  # refinement-6 multimesh, 16 layers: ~10 min, ~30 GB RAM; the fixture holds the
                                                 # 82 prognostic channels of the NEW time slice and, as t_*, the same summaries
                                                 # of the network's tendency (state = x + 0.1 sigma x tendency: a 1e-3 bound on the
@@ -23,11 +25,11 @@ sys.path.insert(0, ROOT)
 import numpy as np, torch
 
 
-def summarise(y):
+def summarise(y, last_row=720):
     y = np.asarray(y, dtype=np.float64)
     blk = y[:, :720].reshape(y.shape[0], 45, 16, 90, 16).mean(axis=(2, 4))
     return dict(y_sample=y[:, ::13, ::17].astype(np.float32), y_block=blk.astype(np.float32),
-                y_last=y[:, 720, ::4].astype(np.float32), y_norm=np.sqrt((y ** 2).sum(axis=(1, 2))),
+                y_last=y[:, last_row, ::4].astype(np.float32), y_norm=np.sqrt((y ** 2).sum(axis=(1, 2))),
                 y_mean=y.mean(axis=(1, 2)), y_std=y.std(axis=(1, 2)))
 
 
@@ -60,6 +62,14 @@ def main(which):
         y = ynew.numpy()[cfg.n_state:cfg.n_state + cfg.n_prog]
         extra = {"t_" + k[2:]: v for k, v in summarise(tend.numpy().T.reshape(cfg.n_prog, cfg.nlat, cfg.nlon)).items()}
         extra["t0"] = np.float64(T0)
+    elif which == "fcn":
+        from skyrim_b200.config import FCN_CHANNELS, fcn_full
+        from skyrim_b200.weights import make_fcn_weights, synthetic_state
+        from oracle.afno_ref import FCNRef
+        cfg = fcn_full()
+        w = make_fcn_weights(cfg, 0)
+        x0 = synthetic_state(FCN_CHANNELS, cfg.nlat, cfg.nlon, 0)
+        y = FCNRef(cfg, w, torch.float32).step(x0).numpy()
     else:
         from skyrim_b200.config import FCNV2_CHANNELS, sfno_full
         from skyrim_b200.weights import make_sfno_weights, synthetic_state
@@ -68,13 +78,13 @@ def main(which):
         w = make_sfno_weights(cfg, 0)
         x0 = synthetic_state(FCNV2_CHANNELS, cfg.nlat, cfg.nlon, 0)
         y = SFNORef(cfg, w, torch.float32).step(x0).numpy()
-    d = summarise(y)
+    d = summarise(y, last_row=y.shape[1] - 1)
     if which == "graphcast":
         d.update(extra)
     d["x0_sample"] = x0[:, ::64, ::64].astype(np.float32)
     d["oracle_seconds"] = np.float64(time.time() - t0)
     d["oracle_threads"] = np.int64(torch.get_num_threads())
-    path = os.path.join(out, f"{which}_721x1440_seed0.npz")
+    path = os.path.join(out, f"{which}_{y.shape[1]}x1440_seed0.npz")
     np.savez_compressed(path, **d)
     print("wrote", path, os.path.getsize(path), "bytes;", f"{time.time() - t0:.1f} s")
 
